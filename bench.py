@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torch.distributed.run)
     python bench.py --impl reference ...                      (optimised CPU restatement of the reference step, host cores)
     python bench.py --workload criteo|multihot|wide           (default criteo = BASELINE.json configs[1] / [2])
+    python bench.py --dump-outputs DIR ...                    (also store what the last timed step computed: see dump_outputs)
 
 Workloads (config.workload), one "step" = ids + forward + sum-reduced sigmoid-CE + backward + all optimizers:
   criteo    configs[1] (N = 1) / configs[2] (N > 1): synthetic Criteo shape, 13 dense + 26 categorical (Criteo-Kaggle
@@ -409,6 +410,35 @@ def parity_check(engine, rows=2048):
             "sample": "%d examples, benchmark model with tables scaled 1e-3, parameters copied from the oracle" % rows}
 
 
+DUMP_BUDGET_BYTES = 56 << 20            # array data of one --dump-outputs directory; with the .npy headers it stays under 64 MB
+
+
+def dump_outputs(model, loss, out_dir):
+    """--dump-outputs: what the timed train step leaves its caller after its last step, as float32 .npy files: `loss.npy` (the
+    step's sum-reduced loss) and every parameter and optimizer slot under its checkpoint key with '/' -> '.' (`<name>.npy`,
+    `<name>.slotN.npy`).  MLP and bias tensors are stored whole; the budget left is shared out over the embedding tables and
+    wide columns, smallest first, and one larger than its share is stored as a fixed sample of its rows, drawn by a generator
+    seeded with the file name, so runs with the same arguments store the same rows.  N > 1: rank 0's replica and row shards."""
+    import zlib
+    from wide_deep_b200.plan import T_EMB_TABLE, T_WIDE_COL
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([loss], dtype=np.float32))
+    arrays = [(name, s) for name in model.tensor_names() for s in range(model.n_slots(name) + 1)]
+    share = {a: int(np.prod(model.plan.local_shape(a[0]))) for a in arrays}
+    tables = sorted((a for a in arrays if model.plan.tensor_names[a[0]][0] in (T_EMB_TABLE, T_WIDE_COL)), key=share.get)
+    left = DUMP_BUDGET_BYTES // 4 - 1 - sum(n for a, n in share.items() if a not in tables)
+    for i, a in enumerate(tables):
+        share[a] = min(share[a], left // (len(tables) - i))
+        left -= share[a]
+    for name, s in arrays:
+        key = name.replace("/", ".") + (".slot%d" % s if s else "")
+        x = model.get_tensor(name, slot=s)
+        if x.size > share[(name, s)]:
+            rows = np.random.default_rng(zlib.crc32(key.encode())).choice(x.shape[0], share[(name, s)] // (x.size // x.shape[0]), replace=False)
+            x = x[np.sort(rows)]
+        np.save(os.path.join(out_dir, key + ".npy"), x)
+
+
 # ------------------------------------------------------------------------------------------------ our arm
 def main():
     ap = argparse.ArgumentParser()
@@ -422,7 +452,13 @@ def main():
                     help="MLP GEMM engine: bf16x3 (tcgen05 kind::f16 on bf16 hi/lo copies, 2^-16 products; re-checked against the "
                          "oracle in this run) | tc3x (tcgen05 kind::tf32 3-pass, 2^-21, the library default) | ffma (fp32 CUDA cores)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss, parameters and optimizer slots of the last one to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs stores what the GPU step computed; the reference arm has nothing to store")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -521,6 +557,10 @@ def main():
     if rank == 0:
         clocks.start()
     ms = timed(step_resident, args.steps)
+    if args.dump_outputs:                                # before the e2e steps train the model further
+        if rank == 0:
+            dump_outputs(model, model.last_loss(), args.dump_outputs)
+        barrier()
     model.prefetch_slot(E2E0, host[0][0])
     for i in range(8):                                   # both e2e slots past their eager steps (graphs captured)
         step_e2e(i)
@@ -667,4 +707,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True                       # the benchmark leaves the tree as it found it
     main()
